@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py -- throughput of the nadavca hot path on B200 (contract: see the task prompt / DESIGN.md "Measurement").
+"""bench.py -- throughput of the nadavca hot path on B200 (DESIGN.md "Measurement").
 
 Workload (BASELINE.json configs[1]): estimate_snps(independent=True) over synthetic reads (~2 kb bases, ~20 k
 samples each, default config: bandwidth 150, min_event_length 2, wobbling, tweak) simulated from the shipped 6-mer
@@ -18,6 +18,8 @@ arms: it is the same scipy call in the reference and here and is not part of the
   --impl reference : the reference's own CPU implementation of the same two DP calls (oracle/_ref = the unmodified
            nadavca C++ compiled by oracle/Makefile; the C port when it is missing) on all host cores, one read per
            worker, on a bounded sample of the same workload.
+  --dump-outputs DIR : after the timed steps, what the last step computed as DIR/<name>.npy (see `dump_outputs`),
+           so that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import json
@@ -56,7 +58,14 @@ def parse_args():
     ap.add_argument('--cpu-sample', type=int, default=0, help='reads in the CPU sample (0 = one per host core)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-overlap', action='store_true', help='accepted for older scripts; no effect')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed as DIR/<name>.npy (at most 64 MB: a fixed, seeded '
+                         'sample of the reads when the batch is larger)')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and (a.impl != 'ours' or a.config not in (1, 2)):
+        ap.error('--dump-outputs applies to the estimate_snps step of --config 1 / 2')
     per_config = {0: (100, 2000, 150), 1: (1000, 2000, 150), 2: (1000, 2000, 150), 3: (62, 100_000, 400),
                   4: (None, 2000, 150)}[a.config]
     a.reads = a.reads if a.reads is not None else per_config[0]
@@ -320,6 +329,59 @@ def workload_config(args, reads_per_gpu):
             'l2': 'inputs larger than L2 (DP matrices of several GB per step)'}
 
 
+# ---- --dump-outputs ------------------------------------------------------------------------------------------------
+
+DUMP_BYTES = 60 << 20        # stays under the 64 MB --dump-outputs promises, .npy headers included
+DUMP_BYTES_PER_ROW = 84      # probabilities 4 x f64 + coverage f32 + log-likelihoods 4 x f64 + events 2 x f64
+DUMP_BYTES_PER_READ = 24     # chunks 3 x f64
+DUMP_SEED = 20_261_020
+
+
+def dump_selection(rows_per_read, budget=DUMP_BYTES):
+    """Indices (ascending) of the reads --dump-outputs writes: all of them when they fit into `budget`, otherwise the
+    longest prefix of one fixed seeded permutation that does, so that runs with the same arguments pick the same
+    reads."""
+    rows = np.asarray(rows_per_read, dtype=np.int64)
+    cost = rows * DUMP_BYTES_PER_ROW + DUMP_BYTES_PER_READ
+    if cost.sum() <= budget:
+        return np.arange(len(rows))
+    order = np.random.default_rng(DUMP_SEED).permutation(len(rows))
+    n = int(np.searchsorted(np.cumsum(cost[order]), budget, side='right'))
+    return np.sort(order[:n])
+
+
+def dump_outputs(out_dir, result, events, log_likelihoods):
+    """What one step of estimate_snps(independent=True) computed, for the reads of `dump_selection` in read order:
+
+      probabilities.npy    float64 (rows, 4)  posterior of A, C, G, T per reference position: the `values` of the
+                                              Chunk objects the call returns, the reads' chunks concatenated
+      coverage.npy         float32 (rows,)    the chunks' `coverage`
+      chunks.npy           float64 (n, 3)     read index, reference start, reference end of each chunk
+      log_likelihoods.npy  float64 (rows, 4)  raw log-likelihoods of estimate_log_likelihoods(wobbling), read
+                                              orientation
+      events.npy           float64 (rows, 2)  event boundaries of refine_alignment(no transitions), relative to the
+                                              start of the read's signal range
+
+    `result` is what ``posterior_stage`` returned; `events` / `log_likelihoods` the per-read arrays of the batches.
+    With several GPUs only rank 0 writes, its own reads."""
+    groups, group_off, probs, cov = result
+    probs, cov = probs.cpu().numpy(), cov.cpu().numpy()
+    keep = dump_selection(np.diff(group_off))
+
+    def rows_of(per_read, width):
+        return np.concatenate([np.zeros((0, width))] + [per_read[i] for i in keep]).astype(np.float64)
+
+    rows = np.concatenate([np.zeros(0, np.int64)] + [np.arange(group_off[i], group_off[i + 1]) for i in keep])
+    out = {'probabilities': probs[rows].astype(np.float64),
+           'coverage': cov[rows].astype(np.float32),
+           'chunks': np.array([(i, groups[i][0], groups[i][1]) for i in keep], dtype=np.float64).reshape(-1, 3),
+           'log_likelihoods': rows_of(log_likelihoods, 4),
+           'events': rows_of(events, 2)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), arr)
+
+
 # ---- GPU arm ------------------------------------------------------------------------------------------------------
 
 def first_read_index(rank, reads_per_gpu):
@@ -413,6 +475,9 @@ def run_ours(args):
     tn, tt = batch_n.timing(), batch_t.timing()
     batch_n.enable_timing(False)
     batch_t.enable_timing(False)
+    if args.dump_outputs and rank == 0:
+        # before the consensus step below, which runs the same batches again
+        dump_outputs(args.dump_outputs, out, batch_n.events()[0], batch_t.log_likelihoods()[0])
     # what the timed steps left resident for the reads of the CPU sample (checked against the reference below)
     n_check = cpu_sample_size(args, len(items)) if (world == 1 and not args.no_cpu_baseline) else 0
     gpu_events = batch_n.events()[0][:n_check] if n_check else []
@@ -513,7 +578,7 @@ def run_ours(args):
     # free the resident batches first: the e2e batch allocates its own workspace
     batch_n.close()
     batch_t.close()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     for _ in range(2):  # warm-up: the first pass also fills the library's device block cache
         e2e_step()
     barrier()

@@ -390,6 +390,35 @@ def test_bench_line_contract():
     assert par['events_compared'] > 0 and par['max_ll_rel'] < 1e-9
 
 
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """bench.py --dump-outputs: float arrays of what the last timed step computed, consistent with each other, under
+    64 MB, and bit-identical between two runs with the same arguments (seeded inputs, deterministic kernels)."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    names = ['chunks', 'coverage', 'events', 'log_likelihoods', 'probabilities']
+    runs = []
+    for tag in ('a', 'b'):
+        out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--reads', '24', '--bases', '400',
+                              '--steps', '2', '--warmup', '1', '--no-api', '--no-consensus', '--no-cpu-baseline',
+                              '--dump-outputs', str(tmp_path / tag)], capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-3000:]
+        assert sorted(os.listdir(tmp_path / tag)) == [n + '.npy' for n in names]
+        assert sum(os.path.getsize(tmp_path / tag / (n + '.npy')) for n in names) <= 64 << 20
+        runs.append({n: np.load(tmp_path / tag / (n + '.npy')) for n in names})
+    d = runs[0]
+    for arr in d.values():
+        assert arr.dtype in (np.float32, np.float64)
+    assert d['chunks'][:, 0].tolist() == list(range(24))  # a small batch is written whole
+    rows = int((d['chunks'][:, 2] - d['chunks'][:, 1]).sum())
+    assert d['probabilities'].shape == d['log_likelihoods'].shape == (rows, 4) and d['events'].shape == (rows, 2)
+    np.testing.assert_allclose(d['probabilities'].sum(axis=1), 1.0, rtol=1e-12)
+    assert np.all(d['coverage'] == 1) and np.all(d['events'][:, 1] - d['events'][:, 0] >= 2)
+    for n in names:
+        assert np.array_equal(runs[0][n], runs[1][n]), n
+
+
 def test_estimator_on_a_non_default_torch_stream(golden_estimator, default_model):
     """The estimator enqueues every kernel on torch's CURRENT stream (PyTorch's side streams are not ordered against
     the legacy default stream): results under ``with torch.cuda.stream(s)`` equal the golden ones."""

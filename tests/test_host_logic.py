@@ -266,6 +266,31 @@ def test_bench_reference_arm_contract():
     assert 'workload' in line['config'] and line['vs_baseline'] is None
 
 
+def test_bench_dump_selection():
+    """--dump-outputs writes every read when the batch fits its budget, otherwise the same seeded sample on every
+    call, within the budget."""
+    import bench
+    rng = np.random.default_rng(5)
+    small = rng.integers(300, 500, size=24)
+    assert bench.dump_selection(small).tolist() == list(range(24))
+    big = rng.integers(1800, 2200, size=1000)
+    keep = bench.dump_selection(big)
+    assert np.array_equal(keep, bench.dump_selection(big.copy()))
+    assert np.all(np.diff(keep) > 0) and 100 < len(keep) < 1000
+    cost = big[keep] * bench.DUMP_BYTES_PER_ROW + bench.DUMP_BYTES_PER_READ
+    assert cost.sum() <= bench.DUMP_BYTES < 64 << 20
+    assert len(bench.dump_selection([bench.DUMP_BYTES])) == 0  # one read larger than the budget: nothing fits
+
+
+def test_bench_rejects_bad_arguments():
+    import subprocess
+    import sys
+    for extra in (['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'unused']):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, capture_output=True, text=True,
+                             timeout=120)
+        assert out.returncode == 2 and 'error' in out.stderr, extra
+
+
 def test_output_writers_keep_the_reference_layout(tmp_path):
     """.npz of `nadavca align` (align_signal.py:83-132) and the SNP table of `nadavca snp` (estimator.py:21-31)."""
     from nadavca_b200 import output
