@@ -12,8 +12,9 @@
 namespace {
 
 // Renormalisation period of the SNP kernel: 16 steps instead of the 8 of the sweeps (dp3.cuh NVB_RENORM_MASK).  A task
-// is a chain of at most 8 lanes, so stale-mantissa slack compounds over at most 8 hops: with <= 2 bits per step and hop
-// (emission mantissa < 2, one addition) 16 steps stay below 2^256, far inside the double range; the sweeps, whose chains
+// is a chain of k+2 lanes, so stale-mantissa slack compounds over at most k+2 hops: with <= 2 bits per step and hop
+// (emission mantissa < 2, one addition) 16 steps stay below 2^(2*16*(k+2)): 2^256 for the 6-mer model, 2^416 at k = 11,
+// inside the double range (2^1022) up to k = 29, beyond any k-mer table that fits a device; the sweeps, whose chains
 // are 32 lanes long, keep 8.  Measured: 71.1 -> 69.8 ms at 1000 reads (the renormalisation was 6.5 % of the kernel's
 // instructions), parity suite and fuzz unchanged (profiles/r02ad).
 #ifndef NVB_SNP_RENORM_MASK
