@@ -1,7 +1,9 @@
 """CPU oracle for the nadavca hot path.   *** TEST INFRASTRUCTURE -- never imported by nadavca_b200 ***
 
 Two back ends behind one interface:
-  * ``port``  -- oracle/libnadavca_oracle.so, the plain-C restatement in oracle/nadavca_oracle.c;
+  * ``port``  -- oracle/libnadavca_oracle.so, the plain-C restatement in oracle/nadavca_oracle.c (``extended``,
+                 oracle/libnadavca_extended.so, restates its EstimateLogLikelihoods in extended precision, see
+                 ``estimate_log_likelihoods_extended``);
   * ``ref``   -- oracle/_ref/dtw*.so, the UNMODIFIED reference C++ compiled by oracle/Makefile (present whenever
                  `make -C oracle ref` ran in a container that has /root/reference; the built file travels to the
                  GPU box).
@@ -226,6 +228,76 @@ def estimate_log_likelihoods(signal, reference, context_before, context_after, a
         _p(cb, ctypes.c_int32), cb.size, _p(ca, ctypes.c_int32), ca.size, _p(anc, ctypes.c_int32), anc.size // 2,
         int(bandwidth), int(min_event_length), int(bool(model_wobbling)), _p(out, ctypes.c_double), *args)
     return (out.tolist(), dbg) if debug else out.tolist()
+
+
+# ---- extended-precision EstimateLogLikelihoods (oracle/nadavca_extended.c) -----------------------------------------
+
+EXT_LIB = os.path.join(HERE, 'libnadavca_extended.so')
+_ext = None
+
+
+def extended_lib():
+    global _ext
+    if _ext is None:
+        if not os.path.exists(EXT_LIB) or os.path.getmtime(EXT_LIB) < os.path.getmtime(
+                os.path.join(HERE, 'nadavca_extended.c')):
+            build('extended')
+        lib = ctypes.CDLL(EXT_LIB)
+        lib.nvx_model_create.restype = ctypes.c_void_p
+        lib.nvx_model_create.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, _f64p, _f64p, ctypes.c_int64]
+        lib.nvx_model_destroy.argtypes = [ctypes.c_void_p]
+        lib.nvx_estimate_log_likelihoods.argtypes = [ctypes.c_void_p, _f64p, ctypes.c_int, _i32p, ctypes.c_int, _i32p,
+                                                     ctypes.c_int, _i32p, ctypes.c_int, _i32p, ctypes.c_int,
+                                                     ctypes.c_int, ctypes.c_int, ctypes.c_int, _f64p, _f64p, _f64p,
+                                                     _f64p, _f64p]
+        _ext = lib
+    return _ext
+
+
+class ExtendedModel:
+    """The model tables of nadavca_extended.c (the reference's double ac / mc, kmer_model.cpp:10-13)."""
+
+    def __init__(self, k, central_position, alphabet_size, mean, sigma):
+        self.k, self.central_position, self.alphabet_size = int(k), int(central_position), int(alphabet_size)
+        self.mean = np.ascontiguousarray(mean, dtype=np.float64)
+        self.sigma = np.ascontiguousarray(sigma, dtype=np.float64)
+        self.handle = ctypes.c_void_p(extended_lib().nvx_model_create(
+            self.k, self.central_position, self.alphabet_size, _p(self.mean, ctypes.c_double),
+            _p(self.sigma, ctypes.c_double), self.mean.size))
+
+    def __del__(self):
+        if getattr(self, 'handle', None):
+            try:
+                extended_lib().nvx_model_destroy(self.handle)
+            except Exception:
+                pass
+            self.handle = None
+
+
+def estimate_log_likelihoods_extended(signal, reference, context_before, context_after, approximate_alignment,
+                                      bandwidth, min_event_length, model, model_wobbling, rows=False):
+    """EstimateLogLikelihoods (dtw.cpp:37-131) in extended precision -> dict with
+      ll     (n, alphabet) log-likelihoods, each rounded once to double;
+      ratio  (n, alphabet) log(L[i][b] / L[i][ref_i]), rounded once (0 on the reference base);
+    and with rows=True also bs, be (band bounds), prefix, suffix (stored rows 0..n packed, as log values) and row_dev
+    (n+1: sum_c P[j][c] S[j][c] relative to row n's, minus 1; the same total for every row in plain mode)."""
+    sig = np.ascontiguousarray(signal, dtype=np.float64)
+    ref, cb, ca, anc = _i32(reference), _i32(context_before), _i32(context_after), _i32(approximate_alignment)
+    a = model.alphabet_size
+    out = {'ll': np.zeros((ref.size, a)), 'ratio': np.zeros((ref.size, a))}
+    extra = [None, None, None]
+    if rows:
+        bs, be = band_bounds(approximate_alignment, sig.size, ref.size, bandwidth)
+        cells = int(np.maximum(be.astype(np.int64) - bs + 1, 0).sum())
+        out.update(bs=bs, be=be, prefix=np.zeros(cells), suffix=np.zeros(cells), row_dev=np.zeros(ref.size + 1))
+        extra = [_p(out['prefix'], ctypes.c_double), _p(out['suffix'], ctypes.c_double),
+                 _p(out['row_dev'], ctypes.c_double)]
+    extended_lib().nvx_estimate_log_likelihoods(
+        model.handle, _p(sig, ctypes.c_double), sig.size, _p(ref, ctypes.c_int32), ref.size, _p(cb, ctypes.c_int32),
+        cb.size, _p(ca, ctypes.c_int32), ca.size, _p(anc, ctypes.c_int32), anc.size // 2, int(bandwidth),
+        int(min_event_length), int(bool(model_wobbling)), _p(out['ll'], ctypes.c_double),
+        _p(out['ratio'], ctypes.c_double), *extra)
+    return out
 
 
 # ---- estimator glue, restated (reference nadavca/estimator.py) -----------------------------------------------
