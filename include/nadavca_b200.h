@@ -63,6 +63,9 @@ void nvb_model_destroy(nvb_model *model);
 int nvb_model_k(const nvb_model *model);                 /* KmerModel::GetK */
 int nvb_model_central_position(const nvb_model *model);  /* KmerModel::GetCentralPosition */
 int nvb_model_alphabet_size(const nvb_model *model);
+/* bytes of device memory held by the model's DP workspaces, summed over every stream it has run on (each workspace
+ * grows to the largest wave seen on its stream and is kept until the model is destroyed, see nvb_batch_refine) */
+int64_t nvb_model_workspace_bytes(const nvb_model *model);
 /* KmerModel::GetExpectedSignal (kmer_model.cpp:32-42), batched; runs as a CUDA kernel.
  * reference/context arrays as in nvb_reads; out has reference_off[n_reads] doubles (host). */
 int nvb_model_expected_signal(nvb_model *model, int32_t n_reads, const int32_t *reference,

@@ -60,6 +60,7 @@ SIGNATURES = {
     'nvb_model_k': (ctypes.c_int, [ctypes.c_void_p]),
     'nvb_model_central_position': (ctypes.c_int, [ctypes.c_void_p]),
     'nvb_model_alphabet_size': (ctypes.c_int, [ctypes.c_void_p]),
+    'nvb_model_workspace_bytes': (ctypes.c_int64, [ctypes.c_void_p]),
     'nvb_model_expected_signal': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, c_i32p, c_i64p, c_i32p, c_i64p,
                                                  c_i32p, c_i64p, c_f64p]),
     'nvb_refine_alignment_batch': (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(NvbReads), ctypes.c_int, c_i32p,

@@ -157,13 +157,13 @@ struct nvb_model {
   int sm_count = 148;
   ModelDev dev{};
   DevBuf<double> mean, ac, mc;
-  std::mutex ws_mutex;
+  mutable std::mutex ws_mutex;
   std::map<cudaStream_t, Workspace> ws;  // std::map: references stay valid while other streams add theirs
   Workspace &workspace(cudaStream_t st) {
     std::lock_guard<std::mutex> lock(ws_mutex);
     return ws[st];
   }
-  size_t workspace_bytes() {
+  size_t workspace_bytes() const {
     std::lock_guard<std::mutex> lock(ws_mutex);
     size_t total = 0;
     for (auto &kv : ws) total += kv.second.bytes();
@@ -316,6 +316,7 @@ void nvb_model_destroy(nvb_model *model) {
 int nvb_model_k(const nvb_model *m) { return m ? m->dev.k : 0; }
 int nvb_model_central_position(const nvb_model *m) { return m ? m->dev.central : 0; }
 int nvb_model_alphabet_size(const nvb_model *m) { return m ? m->dev.alphabet : 0; }
+int64_t nvb_model_workspace_bytes(const nvb_model *m) { return m ? (int64_t)m->workspace_bytes() : 0; }
 
 }  // extern "C"
 

@@ -197,8 +197,13 @@ class ProbabilityEstimator:
         The reads are cut into sub-batches of ``sub_batch_reads`` (config key, default 256), each on its own CUDA
         stream (per-stream DP workspaces, csrc/api.cu), so that the host work between the two DP calls -- D2H of the
         event means, the FITPACK spline fits (worker processes), H2D of the splines -- of one sub-batch overlaps the
-        kernels of the others."""
-        import torch
+        kernels of the others.
+
+        The model keeps one DP workspace per stream until it is destroyed, so the sub-batch streams are created once
+        per device and process (``_sub_batch_streams``) and reused by every call and every estimator: a process that
+        calls this over and over holds at most four sub-batch workspaces per model, not one per stream torch hands
+        out.  Work on a caller's own current stream (a single sub-batch runs there) is the caller's business: every
+        distinct stream a caller runs on keeps its own workspace."""
         from .read import fit_splines_async
         items = [it for it in (self._prepare(read, reference) for read in reads) if it is not None]
         if not items:
@@ -207,8 +212,7 @@ class ProbabilityEstimator:
         per = max(1, int(self.sub_batch_reads))
         n_sub = -(-len(items) // per)
         bounds = [len(items) * j // n_sub for j in range(n_sub + 1)]
-        streams = [torch.cuda.Stream(device=_device(self.kmer_model)) for _ in range(min(n_sub, 4))] if n_sub > 1 \
-            else [main]
+        streams = _sub_batch_streams(_device(self.kmer_model), min(n_sub, 4)) if n_sub > 1 else [main]
         subs = []
         for j in range(n_sub):
             sub_items = items[bounds[j]:bounds[j + 1]]
@@ -537,6 +541,20 @@ def _current_stream(kmer_model):
     be used under ``with torch.cuda.stream(s)``)."""
     import torch
     return torch.cuda.current_stream(_device(kmer_model))
+
+
+_SUB_BATCH_STREAMS = {}
+
+
+def _sub_batch_streams(dev, count):
+    """The first `count` sub-batch streams of device `dev`, created on first use and kept for the process
+    (``torch.cuda.Stream()`` hands out a different pooled stream on every call, and each new stream would cost the
+    model a new DP workspace)."""
+    import torch
+    cache = _SUB_BATCH_STREAMS.setdefault(dev.index, [])
+    while len(cache) < count:
+        cache.append(torch.cuda.Stream(device=dev))
+    return cache[:count]
 
 
 def _device(kmer_model):
