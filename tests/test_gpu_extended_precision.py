@@ -171,7 +171,7 @@ def _check_read(res, truth, N, n, ref, term):
     fin = np.isfinite(truth['ll'])
     if not np.array_equal(np.isfinite(res), fin):
         bad = np.argwhere(np.isfinite(res) != fin)[0]
-        return np.inf, np.inf, 'finite pattern differs first at (%d, %d)' % tuple(bad)
+        return np.inf, np.inf, np.inf, 'finite pattern differs first at (%d, %d)' % tuple(bad)
     tot_err = abs(res[0, ref[0]] - truth['ll'][0, ref[0]]) / bar if fin[0, ref[0]] else 0.0
     rows = np.arange(n)
     gr = res - res[rows, ref][:, None]
