@@ -47,8 +47,7 @@ int nvb_device_count(void);
 int nvb_trim_memory(int device);
 /* Schedule of the forward / backward row sweeps (a tuning knob without a reference counterpart; results are
  * identical): AUTO picks per wave by batch size, ROTATE = one rotating wavefront per (read, direction), STRIPES =
- * pipelined 31-row stripes.  The environment variable NVB_SWEEP=r|s sets the initial value when the library is
- * loaded.  Returns the previous setting. */
+ * pipelined 31-row stripes.  Returns the previous setting. */
 #define NVB_SWEEP_AUTO 0
 #define NVB_SWEEP_ROTATE 1
 #define NVB_SWEEP_STRIPES 2
@@ -109,8 +108,6 @@ int nvb_estimate_log_likelihoods_batch(nvb_model *model, const nvb_reads *reads,
 /* Upload a batch and compute its band geometry (ComputeBandStarts/Ends dtw.cpp:7-35) on the device. */
 nvb_batch *nvb_batch_create(nvb_model *model, const nvb_reads *reads);
 void nvb_batch_destroy(nvb_batch *batch);
-/* replace the signal values (same offsets), e.g. after Read.tweak_signal_normalization (estimator.py:96-97) */
-int nvb_batch_set_signal(nvb_batch *batch, const double *signal);
 /* limit for the DP matrices kept in HBM at one time (bytes; 0 = 70% of the free device memory).  Batches that
  * need more are processed in several waves of reads. */
 int nvb_batch_set_workspace_limit(nvb_batch *batch, int64_t bytes);
@@ -129,11 +126,6 @@ int nvb_batch_get_bands(nvb_batch *batch, int32_t *starts, int32_t *ends);
 /* DP cell counts of the batch by the formulas of SURVEY.md 8(d): [0] refine with transitions, [1] refine without,
  * [2] estimate forward+backward, [3] estimate SNP loop */
 int nvb_batch_cell_counts(nvb_batch *batch, int model_wobbling, int64_t counts[4]);
-/* device pointers of resident results (valid until the next run / destroy): raw log-likelihoods
- * double[sum n][alphabet], events int32[sum n][2], status int32[n_reads] */
-double *nvb_batch_d_log_likelihoods(nvb_batch *batch);
-int32_t *nvb_batch_d_events(nvb_batch *batch);
-int32_t *nvb_batch_d_status(nvb_batch *batch);
 /* debugging aid: the stored DP rows of read `read` after nvb_batch_estimate (plane 0 = prefix, 1 = suffix) as
  * log-probabilities, packed band rows 0..n (cells = sum of band widths); the read must be in the last wave */
 int nvb_batch_debug_rows(nvb_batch *batch, int read, int plane, double *out_log, int64_t n_cells);
@@ -166,17 +158,14 @@ int nvb_batch_event_means(nvb_batch *batch, double *out);
  * spline_off[r+1] - spline_off[r] per read (0 = leave the read's signal as it is); degree = 3 for the reference. */
 int nvb_batch_apply_splines(nvb_batch *batch, const double *knots, const double *coefs, const int64_t *spline_off,
                             int degree, void *stream);
-/* the resident signal values (after nvb_batch_set_signal / nvb_batch_apply_splines), double[signal_off[n_reads]] */
+/* the resident signal values (after nvb_batch_apply_splines), double[signal_off[n_reads]] */
 int nvb_batch_get_signal(nvb_batch *batch, double *out);
 /* _normalize_log_likelihoods + reverse-strand complement/flip (estimator.py:45-47,111-119) applied to the
  * resident raw log-likelihoods; d_chunks: double[sum n][4] device buffer (alphabet must be 4).  Asynchronous: the
- * per-read `reverse` (and `dest` below) arrays are kept on the device and re-uploaded only when they change. */
+ * per-read `reverse` (and `dest` of nvb_batch_scatter_add_rows) arrays are kept on the device and re-uploaded only
+ * when they change. */
 int nvb_batch_chunk_values(nvb_batch *batch, const int32_t *reverse, double normalization_event_length,
                            double *d_chunks, void *stream);
-/* consensus accumulation (estimator.py:226-231): d_acc[dest[r] + i][j] += chunk_r[i][j], d_cov[dest[r]+i] += 1
- * for every read r with dest[r] >= 0 and status OK.  dest is a HOST array of n_reads row offsets. */
-int nvb_batch_scatter_add(nvb_batch *batch, const double *d_chunks, const int64_t *dest, double *d_acc,
-                          int32_t *d_cov, void *stream);
 /* ---- batched anchor construction: replaces the per-read CIGAR walk and signal-alignment glue of
  * ApproximateAligner (alignment.py:109-140 parse the CIGAR and keep matching bases; alignment.py:142-186 convert them
  * to signal anchors and ranges).  Mapping the reads (BWA) stays on the host; its hits come in as CSR arrays. ---------- */
@@ -222,25 +211,19 @@ int nvb_normalize_clip_d(int device, const double *d_values, int64_t n, double s
 
 /* Consensus accumulator as ROWS of 5 doubles [sum A, sum C, sum G, sum T, coverage] (estimator.py:226-231): sums and
  * coverage travel in one buffer, so the exchange between GPUs is one collective (reduce-scatter by genome slice, or
- * all-reduce).  d_rows is a zero-initialised device buffer of (total rows, 5) doubles; dest as in
- * nvb_batch_scatter_add. */
+ * all-reduce).  d_rows is a zero-initialised device buffer of (total rows, 5) doubles: d_rows[dest[r] + i][j] +=
+ * chunk_r[i][j] and d_rows[dest[r] + i][4] += 1 for every read r with dest[r] >= 0 and status OK.  dest is a HOST
+ * array of n_reads row offsets. */
 int nvb_batch_scatter_add_rows(nvb_batch *batch, const double *d_chunks, const int64_t *dest, double *d_rows,
                                void *stream);
 /* _compute_posterior (estimator.py:123-156) for the global rows [row_lo, row_hi) of the concatenated groups, from
  * consensus rows that start at global row base_row (a rank's slice plus its k-1 halo rows); d_ref and d_group_off
- * are indexed by global rows.  d_out_rows: (row_hi - row_lo, 5) doubles = [P(A), P(C), P(G), P(T), coverage].  Only
- * enqueues the kernel on `stream`. */
+ * are indexed by global rows, d_ref int8 (0..3, anything else = no base matches), d_group_off int64[n_groups+1].
+ * d_out_rows: (row_hi - row_lo, 5) doubles = [P(A), P(C), P(G), P(T), coverage].  Only enqueues the kernel on
+ * `stream`. */
 int nvb_posterior_rows_d(int device, const double *d_rows, int64_t base_row, int64_t row_lo, int64_t row_hi,
                          const int8_t *d_ref, const int64_t *d_group_off, int32_t n_groups, int k, double snp_prior,
                          double *d_out_rows, void *stream);
-/* _compute_posterior (estimator.py:123-156) over concatenated groups: d_ll double[total][4], d_ref int8[total]
- * (0..3, anything else = no base matches), group_off HOST int64[n_groups+1]; d_out double[total][4]. */
-int nvb_posterior(int device, const double *d_ll, const int8_t *d_ref, const int64_t *group_off,
-                  int32_t n_groups, int k, double snp_prior, double *d_out, void *stream);
-/* the same with the group offsets already on the device (int64[n_groups+1], total = d_group_off[n_groups]): no upload
- * and no synchronisation, the call only enqueues the kernel on `stream` */
-int nvb_posterior_d(int device, const double *d_ll, const int8_t *d_ref, const int64_t *d_group_off,
-                    int32_t n_groups, int64_t total, int k, double snp_prior, double *d_out, void *stream);
 
 #ifdef __cplusplus
 }

@@ -69,7 +69,6 @@ SIGNATURES = {
                                                           c_f64p, c_i32p]),
     'nvb_batch_create': (ctypes.c_void_p, [ctypes.c_void_p, ctypes.POINTER(NvbReads)]),
     'nvb_batch_destroy': (None, [ctypes.c_void_p]),
-    'nvb_batch_set_signal': (ctypes.c_int, [ctypes.c_void_p, c_f64p]),
     'nvb_batch_set_workspace_limit': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64]),
     'nvb_batch_refine': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]),
     'nvb_batch_estimate': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]),
@@ -77,9 +76,6 @@ SIGNATURES = {
     'nvb_batch_get_log_likelihoods': (ctypes.c_int, [ctypes.c_void_p, c_f64p, c_i32p]),
     'nvb_batch_get_bands': (ctypes.c_int, [ctypes.c_void_p, c_i32p, c_i32p]),
     'nvb_batch_cell_counts': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, c_i64p]),
-    'nvb_batch_d_log_likelihoods': (ctypes.c_void_p, [ctypes.c_void_p]),
-    'nvb_batch_d_events': (ctypes.c_void_p, [ctypes.c_void_p]),
-    'nvb_batch_d_status': (ctypes.c_void_p, [ctypes.c_void_p]),
     'nvb_batch_launch_count': (ctypes.c_int64, [ctypes.c_void_p]),
     'nvb_batch_debug_rows': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, c_f64p, ctypes.c_int64]),
     'nvb_batch_enable_timing': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
@@ -91,8 +87,6 @@ SIGNATURES = {
     'nvb_batch_get_signal': (ctypes.c_int, [ctypes.c_void_p, c_f64p]),
     'nvb_batch_chunk_values': (ctypes.c_int, [ctypes.c_void_p, c_i32p, ctypes.c_double, ctypes.c_void_p,
                                               ctypes.c_void_p]),
-    'nvb_batch_scatter_add': (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, c_i64p, ctypes.c_void_p,
-                                             ctypes.c_void_p, ctypes.c_void_p]),
     'nvb_signal_anchors_batch': (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(NvbHits), c_i32p, c_i64p,
                                                 ctypes.c_void_p]),
     'nvb_radix_histogram_d': (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
@@ -108,11 +102,6 @@ SIGNATURES = {
     'nvb_posterior_rows_d': (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64,
                                             ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
                                             ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
-    'nvb_posterior': (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, c_i64p, ctypes.c_int32,
-                                     ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
-    'nvb_posterior_d': (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
-                                       ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p,
-                                       ctypes.c_void_p]),
 }
 
 _lib = None

@@ -3,7 +3,6 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -20,19 +19,7 @@ namespace {
 thread_local std::string g_err;
 thread_local int g_code = 0;  // code of the last failure on this thread (what the one-shot calls return)
 
-// Tuning / debugging switches: the environment is read ONCE, when the library is loaded; nvb_set_sweep_schedule
-// changes the schedule at run time (tests force both schedules through it).
-struct Options {
-  int sweep = NVB_SWEEP_AUTO;   // NVB_SWEEP=r|s
-  bool skip_path = false;       // NVB_DEBUG_SKIP_PATH: keep the prefix plane for nvb_batch_debug_rows
-  int sweep_warps = 0;          // NVB_SWEEP_WARPS: warps per (read, direction) of the striped sweep, 0 = automatic
-  Options() {
-    if (const char *env = getenv("NVB_SWEEP")) sweep = env[0] == 'r' ? NVB_SWEEP_ROTATE : (env[0] == 's' ? NVB_SWEEP_STRIPES : NVB_SWEEP_AUTO);
-    skip_path = getenv("NVB_DEBUG_SKIP_PATH") != nullptr;
-    if (const char *env = getenv("NVB_SWEEP_WARPS")) sweep_warps = atoi(env);
-  }
-};
-Options g_opt;
+int g_sweep = NVB_SWEEP_AUTO;  // sweep schedule, set by nvb_set_sweep_schedule (tests force both schedules through it)
 
 int fail(int code, const char *fmt, ...) {
   char buf[512];
@@ -250,8 +237,8 @@ int nvb_abi_version(void) { return 1; }
 const char *nvb_last_error(void) { return g_err.c_str(); }
 
 int nvb_set_sweep_schedule(int schedule) {
-  const int before = g_opt.sweep;
-  if (schedule == NVB_SWEEP_AUTO || schedule == NVB_SWEEP_ROTATE || schedule == NVB_SWEEP_STRIPES) g_opt.sweep = schedule;
+  const int before = g_sweep;
+  if (schedule == NVB_SWEEP_AUTO || schedule == NVB_SWEEP_ROTATE || schedule == NVB_SWEEP_STRIPES) g_sweep = schedule;
   return before;
 }
 
@@ -298,7 +285,6 @@ nvb_model *nvb_model_create(int k, int central_position, int alphabet_size, cons
   }
   m->dev.k = k; m->dev.central = central_position; m->dev.alphabet = alphabet_size; m->dev.n_kmers = n_kmers;
   m->dev.mean = m->mean.p; m->dev.ac = m->ac.p; m->dev.mc = m->mc.p;
-  m->dev.log_p_in = log(0.01);
   return m;
 }
 
@@ -439,15 +425,15 @@ int run_sweep(nvb_batch *b, Workspace &ws, int mode, const Wave &w, cudaStream_t
   const int items = 2 * (w.b1 - w.b0);
   const int resident = b->model->sm_count * 16;  // sweep warps of one resident wave
   bool rotate = w.maxw <= 640 && (w.maxw <= 352 || mode == NVB_MODE_PLAIN || 4 * items >= resident);
-  if (g_opt.sweep != NVB_SWEEP_AUTO) rotate = w.maxw <= 640 && g_opt.sweep == NVB_SWEEP_ROTATE;
+  if (g_sweep != NVB_SWEEP_AUTO) rotate = w.maxw <= 640 && g_sweep == NVB_SWEEP_ROTATE;
   for (int i = w.b0; i < w.b1 && rotate; i++) rotate = !b->no_rotation[i];
   if (rotate)
     return nvbk_sweep_rotate(M, b->dev, mode, w.b0, w.b1, b->d_mat_base.p, ws.pF.p, ws.pX.p, ws.sF.p, ws.sX.p, st);
   // band rows too wide for the shared-memory hand-off rows of the striped sweep go through global scratch rows
-  const int64_t need = nvbk_sweep2_global_handoff_doubles(mode, w.b1 - w.b0, w.maxw, g_opt.sweep_warps);
+  const int64_t need = nvbk_sweep2_global_handoff_doubles(mode, w.b1 - w.b0, w.maxw);
   if (need > 0 && ws.handoff.alloc((size_t)need, st, true) != cudaSuccess) { cudaGetLastError(); return -2; }
-  return nvbk_sweep2(M, b->dev, mode, w.b0, w.b1, w.maxw, g_opt.sweep_warps, b->d_mat_base.p, ws.pF.p, ws.pX.p, ws.sF.p,
-                     ws.sX.p, need > 0 ? ws.handoff.p : nullptr, st);
+  return nvbk_sweep2(M, b->dev, mode, w.b0, w.b1, w.maxw, b->d_mat_base.p, ws.pF.p, ws.pX.p, ws.sF.p, ws.sX.p,
+                     need > 0 ? ws.handoff.p : nullptr, st);
 }
 
 int64_t matrix_cells(const nvb_batch *b, int i, int mode) {
@@ -584,15 +570,6 @@ int nvb_trim_memory(int device) {
   return NVB_OK;
 }
 
-int nvb_batch_set_signal(nvb_batch *b, const double *signal) {
-  if (!b || !signal) return fail(NVB_EINVAL, "nvb_batch_set_signal: NULL argument");
-  CU(cudaSetDevice(b->model->device));
-  b->drain();  // earlier runs may still be reading the old values
-  CU(cudaMemcpyAsync(b->d_signal.p, signal, (size_t)b->total_sig * sizeof(double), cudaMemcpyHostToDevice, b->run_stream));
-  CU(cudaStreamSynchronize(b->run_stream));
-  return NVB_OK;
-}
-
 int nvb_batch_set_workspace_limit(nvb_batch *b, int64_t bytes) {
   if (!b) return fail(NVB_EINVAL, "NULL batch");
   b->ws_limit = bytes;
@@ -618,15 +595,14 @@ int nvb_batch_refine(nvb_batch *b, int model_transitions, void *stream) {
       if (src == -1) return fail(NVB_EINVAL, "min_event_length %d is not supported (maximum 6)", b->dev.mel);
       if (src) return fail(NVB_ENOMEM, "cannot allocate the hand-off rows of the sweep for a band row of %d columns", w.maxw);
     }
-    if (!g_opt.skip_path) {  // debugging aid: keep the prefix plane for nvb_batch_debug_rows
+    {
       StageTimer t(b, 1, st);
       nvbk_score(w.cells, ws.pF.p, ws.pX.p, ws.sF.p, ws.sX.p, st);
       if (nvbk_path2(b->dev, mode, w.b0, w.b1, b->path_pk, b->d_mat_base.p, ws.pF.p, ws.records.p, b->d_rec_base.p,
                      ws.dp.p, b->d_dp_base.p, w.maxw, b->d_events.p, b->d_status.p, st))
         return fail(NVB_ECUDA, "path kernel: cannot reserve shared memory");
     }
-    b->launches += 1;
-    b->launches += 2;
+    b->launches += 3;
   }
   CU(cudaGetLastError());
   b->have_events = true;
@@ -742,9 +718,6 @@ int nvb_batch_cell_counts(nvb_batch *b, int model_wobbling, int64_t counts[4]) {
   return NVB_OK;
 }
 
-double *nvb_batch_d_log_likelihoods(nvb_batch *b) { return b && b->have_ll ? b->d_ll.p : nullptr; }
-int32_t *nvb_batch_d_events(nvb_batch *b) { return b && b->have_events ? b->d_events.p : nullptr; }
-int32_t *nvb_batch_d_status(nvb_batch *b) { return b ? b->d_status.p : nullptr; }
 int64_t nvb_batch_launch_count(const nvb_batch *b) { return b ? b->launches : 0; }
 
 int nvb_batch_debug_rows(nvb_batch *b, int read, int plane, double *out_log, int64_t n_cells) {
@@ -947,25 +920,6 @@ int nvb_batch_chunk_values(nvb_batch *b, const int32_t *reverse, double normaliz
   return NVB_OK;
 }
 
-int nvb_batch_scatter_add(nvb_batch *b, const double *d_chunks, const int64_t *dest, double *d_acc, int32_t *d_cov,
-                          void *stream) {
-  if (!b || !d_chunks || !dest || !d_acc || !d_cov) return fail(NVB_EINVAL, "NULL argument");
-  CU(cudaSetDevice(b->model->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  b->touch(st);
-  const size_t n = (size_t)b->n_reads;
-  if (b->h_dest.size() != n || !std::equal(dest, dest + n, b->h_dest.begin())) {
-    CU(cudaStreamSynchronize(st));
-    b->h_dest.assign(dest, dest + n);
-    CU(upload(b->d_dest, b->h_dest.data(), n, st));
-    CU(cudaStreamSynchronize(st));
-  }
-  nvbk_scatter_add(b->dev, d_chunks, b->d_dest.p, b->d_status.p, b->total_ref, d_acc, d_cov, st);
-  b->launches++;
-  CU(cudaGetLastError());
-  return NVB_OK;
-}
-
 int nvb_signal_anchors_batch(int device, const nvb_hits *h, int32_t *anchors, int64_t *meta, void *stream) {
   if (!h || !anchors || !meta || h->n_reads < 0) return fail(NVB_EINVAL, "NULL argument");
   if (nvb_device_count() <= device) return fail(NVB_ECUDA, "CUDA device %d not available (no CPU fallback)", device);
@@ -1082,30 +1036,6 @@ int nvb_posterior_rows_d(int device, const double *d_rows, int64_t base_row, int
   nvbk_posterior_rows(d_rows, base_row, row_lo, row_hi, d_ref, d_group_off, n_groups, k, snp_prior, d_out_rows,
                       (cudaStream_t)stream);
   CU(cudaGetLastError());
-  return NVB_OK;
-}
-
-int nvb_posterior_d(int device, const double *d_ll, const int8_t *d_ref, const int64_t *d_group_off, int32_t n_groups,
-                    int64_t total, int k, double snp_prior, double *d_out, void *stream) {
-  if (!d_ll || !d_ref || !d_group_off || !d_out || n_groups < 0 || total < 0) return fail(NVB_EINVAL, "bad argument");
-  if (nvb_device_count() <= device) return fail(NVB_ECUDA, "CUDA device %d not available (no CPU fallback)", device);
-  CU(cudaSetDevice(device));
-  nvbk_posterior(d_ll, d_ref, d_group_off, n_groups, total, k, snp_prior, d_out, (cudaStream_t)stream);
-  CU(cudaGetLastError());
-  return NVB_OK;
-}
-
-int nvb_posterior(int device, const double *d_ll, const int8_t *d_ref, const int64_t *group_off, int32_t n_groups,
-                  int k, double snp_prior, double *d_out, void *stream) {
-  if (!d_ll || !d_ref || !group_off || !d_out || n_groups < 0) return fail(NVB_EINVAL, "bad argument");
-  if (nvb_device_count() <= device) return fail(NVB_ECUDA, "CUDA device %d not available (no CPU fallback)", device);
-  CU(cudaSetDevice(device));
-  cudaStream_t st = (cudaStream_t)stream;
-  DevBuf<int64_t> d_goff;
-  CU(upload(d_goff, group_off, (size_t)n_groups + 1, st));
-  nvbk_posterior(d_ll, d_ref, d_goff.p, n_groups, group_off[n_groups], k, snp_prior, d_out, st);
-  CU(cudaGetLastError());
-  CU(cudaStreamSynchronize(st));
   return NVB_OK;
 }
 

@@ -143,18 +143,6 @@ __global__ void chunk_values_kernel(BatchDev B, const double *ll, const int32_t 
   }
 }
 
-__global__ void scatter_add_kernel(BatchDev B, const double *chunks, const int64_t *dest, const int32_t *status,
-                                   int64_t total, double *acc, int32_t *cov) {
-  int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (g >= total) return;
-  const int b = find_read(B, g);
-  if (dest[b] < 0 || status[b] != 0) return;
-  const int64_t p = dest[b] + (g - B.ref_off[b]);
-#pragma unroll
-  for (int j = 0; j < 4; j++) atomicAdd(acc + p * 4 + j, chunks[g * 4 + j]);
-  atomicAdd(cov + p, 1);
-}
-
 // Consensus accumulator as ROWS of 5 doubles [A, C, G, T, coverage]: the sums of estimator.py:226-231 and the coverage
 // count of estimator.py:229-230 in one buffer, so that the exchange between GPUs is ONE collective (coverage counts
 // are small integers, exact in a double).
@@ -171,9 +159,9 @@ __global__ void scatter_add_rows_kernel(BatchDev B, const double *chunks, const 
 }
 
 // _compute_posterior (estimator.py:131-156) at global row g: window [max(0,i-k+1), min(i+k,L)) inside the position's
-// group, same accumulation order as the reference.  `ll` holds rows of `ld` doubles starting at global row `base`
-// (ld = 4, base = 0: a plain (total, 4) matrix; ld = 5: a slice of the consensus rows with its k-1 halo rows).
-__device__ __forceinline__ void posterior_at(const double *ll, int ld, int64_t base, const int8_t *ref,
+// group, same accumulation order as the reference.  `rows` holds consensus rows of 5 doubles starting at global row
+// `base` (the whole buffer, or a slice with its k-1 halo rows).
+__device__ __forceinline__ void posterior_at(const double *rows, int64_t base, const int8_t *ref,
                                              const int64_t *group_off, int n_groups, int64_t g, int k, double snp_prior,
                                              double pr_out[4]) {
   int lo = 0, hi = n_groups;
@@ -184,10 +172,10 @@ __device__ __forceinline__ void posterior_at(const double *ll, int ld, int64_t b
   const int64_t gs = group_off[lo], ge = group_off[lo + 1];
   const int64_t i = g - gs, L = ge - gs;
   const int64_t cs = max((int64_t)0, i - k + 1), ce = min(i + k, L);
-  const double *row0 = ll + (gs - base) * ld;  // row of the group's first position
+  const double *row0 = rows + (gs - base) * 5;  // row of the group's first position
   double mx = nvb_neg_inf();
   for (int64_t i2 = cs; i2 < ce; i2++)
-    for (int j = 0; j < 4; j++) mx = fmax(mx, row0[i2 * ld + j]);
+    for (int j = 0; j < 4; j++) mx = fmax(mx, row0[i2 * 5 + j]);
   // _corrected_priors (estimator.py:123-129)
   const double c = 3.0;
   const double p1 = 1 - snp_prior, p2 = snp_prior / c;
@@ -197,14 +185,14 @@ __device__ __forceinline__ void posterior_at(const double *ll, int ld, int64_t b
   const int rb = ref[g];
   for (int j = 0; j < 4; j++) {
     const double prior = (j != rb) ? snp_h : nonsnp_h;
-    double v = exp(row0[i * ld + j] - mx) * prior;
+    double v = exp(row0[i * 5 + j] - mx) * prior;
     if (j == rb) {
       for (int64_t i2 = cs; i2 < ce; i2++) {
         if (i2 == i) continue;
         const int rb2 = ref[gs + i2];
         for (int j2 = 0; j2 < 4; j2++) {
           if (j2 == rb2) continue;
-          v += exp(row0[i2 * ld + j2] - mx) * snp_h;
+          v += exp(row0[i2 * 5 + j2] - mx) * snp_h;
         }
       }
     }
@@ -215,15 +203,6 @@ __device__ __forceinline__ void posterior_at(const double *ll, int ld, int64_t b
   for (int j = 0; j < 4; j++) pr_out[j] = pr[j] / sum;
 }
 
-__global__ void posterior_kernel(const double *ll, const int8_t *ref, const int64_t *group_off, int n_groups,
-                                 int64_t total, int k, double snp_prior, double *out) {
-  int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (g >= total) return;
-  double pr[4];
-  posterior_at(ll, 4, 0, ref, group_off, n_groups, g, k, snp_prior, pr);
-  for (int j = 0; j < 4; j++) out[g * 4 + j] = pr[j];
-}
-
 // Posterior of the global rows [row_lo, row_hi) from consensus rows of 5 doubles that start at global row `base`
 // (base <= row_lo - (k-1) unless row_lo opens a group): out rows of 5 = [P(A), P(C), P(G), P(T), coverage].
 __global__ void posterior_rows_kernel(const double *rows, int64_t base, int64_t row_lo, int64_t row_hi,
@@ -232,7 +211,7 @@ __global__ void posterior_rows_kernel(const double *rows, int64_t base, int64_t 
   int64_t g = row_lo + blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (g >= row_hi) return;
   double pr[4];
-  posterior_at(rows, 5, base, ref, group_off, n_groups, g, k, snp_prior, pr);
+  posterior_at(rows, base, ref, group_off, n_groups, g, k, snp_prior, pr);
   double *o = out + (g - row_lo) * 5;
   for (int j = 0; j < 4; j++) o[j] = pr[j];
   o[4] = rows[(g - base) * 5 + 4];
@@ -275,19 +254,6 @@ void nvbk_apply_splines(const BatchDev &B, double *d_signal, const double *d_kno
 void nvbk_chunk_values(const BatchDev &B, const double *d_ll, const int32_t *d_reverse, double nel, int64_t total,
                        double *d_chunks, cudaStream_t st) {
   if (total > 0) chunk_values_kernel<<<blocks_for(total), 256, 0, st>>>(B, d_ll, d_reverse, nel, total, d_chunks);
-}
-
-void nvbk_scatter_add(const BatchDev &B, const double *d_chunks, const int64_t *d_dest, const int32_t *d_status,
-                      int64_t total, double *d_acc, int32_t *d_cov, cudaStream_t st) {
-  if (total > 0)
-    scatter_add_kernel<<<blocks_for(total), 256, 0, st>>>(B, d_chunks, d_dest, d_status, total, d_acc, d_cov);
-}
-
-void nvbk_posterior(const double *d_ll, const int8_t *d_ref, const int64_t *d_group_off, int n_groups,
-                    int64_t total, int k, double snp_prior, double *d_out, cudaStream_t st) {
-  if (total > 0)
-    posterior_kernel<<<blocks_for(total), 256, 0, st>>>(d_ll, d_ref, d_group_off, n_groups, total, k, snp_prior,
-                                                        d_out);
 }
 
 void nvbk_scatter_add_rows(const BatchDev &B, const double *d_chunks, const int64_t *d_dest, const int32_t *d_status,

@@ -14,8 +14,8 @@ void nvbk_expected_signal(const ModelDev &M, const BatchDev &B, int64_t total, d
 // row of the wave.  Returns -1 for an unsupported min_event_length, -2 when the hand-off rows do not fit shared memory.
 // g_handoff: global scratch for the hand-off rows of band rows too wide for shared memory (size from
 // nvbk_sweep2_global_handoff_doubles, 0 = not needed).
-int64_t nvbk_sweep2_global_handoff_doubles(int mode, int n_reads, int wave_maxw, int force_warps);
-int nvbk_sweep2(const ModelDev &M, const BatchDev &B, int mode, int b0, int b1, int wave_maxw, int force_warps,
+int64_t nvbk_sweep2_global_handoff_doubles(int mode, int n_reads, int wave_maxw);
+int nvbk_sweep2(const ModelDev &M, const BatchDev &B, int mode, int b0, int b1, int wave_maxw,
                 const int64_t *d_mat_base, double *pF, int32_t *pX, double *sF, int32_t *sX, double *g_handoff,
                 cudaStream_t st);
 // rows5.cu: the same rows with one continuously rotating wavefront per (read, direction); for reads whose bands allow
@@ -50,10 +50,6 @@ void nvbk_apply_splines(const BatchDev &B, double *d_signal, const double *d_kno
                         const int64_t *d_spl_off, int degree, int64_t total, cudaStream_t st);
 void nvbk_chunk_values(const BatchDev &B, const double *d_ll, const int32_t *d_reverse, double nel, int64_t total,
                        double *d_chunks, cudaStream_t st);
-void nvbk_scatter_add(const BatchDev &B, const double *d_chunks, const int64_t *d_dest, const int32_t *d_status,
-                      int64_t total, double *d_acc, int32_t *d_cov, cudaStream_t st);
-void nvbk_posterior(const double *d_ll, const int8_t *d_ref, const int64_t *d_group_off, int n_groups,
-                    int64_t total, int k, double snp_prior, double *d_out, cudaStream_t st);
 void nvbk_scatter_add_rows(const BatchDev &B, const double *d_chunks, const int64_t *d_dest, const int32_t *d_status,
                            int64_t total, double *d_rows, cudaStream_t st);
 void nvbk_posterior_rows(const double *d_rows, int64_t base, int64_t row_lo, int64_t row_hi, const int8_t *d_ref,

@@ -383,13 +383,12 @@ struct SweepPlan {
   bool global_handoff;
 };
 
-SweepPlan plan_sweep(int mode, int wave_maxw, int force_warps) {
+SweepPlan plan_sweep(int mode, int wave_maxw) {
   SweepPlan p;
   // warps per (read, direction): a stripe lasts ~W + 12*31 steps, a new one can start every ~11*31 steps
   p.width = (wave_maxw + 1) & ~1;  // keeps the int32 plane 8-byte aligned
   int NW = (wave_maxw + 12 * PAIRS + 11 * PAIRS - 1) / (11 * PAIRS);
   NW = NW < 1 ? 1 : (NW > 7 ? 7 : NW);
-  if (force_warps > 0) NW = force_warps > 7 ? 7 : force_warps;  // experiments (NVB_SWEEP_WARPS, read at load)
   const int tiles_per_warp = (mode == NVB_MODE_TRANS) ? 2 : 1;
   auto tile_bytes = [&](int nw) { return (size_t)64 + 16 + (size_t)nw * (tiles_per_warp * kTileBytes + kRingStride); };
   auto bytes = [&](int nw) { return tile_bytes(nw) + (size_t)(nw + 1) * p.width * (sizeof(double) + sizeof(int32_t)); };
@@ -407,19 +406,19 @@ SweepPlan plan_sweep(int mode, int wave_maxw, int force_warps) {
 double nvbk_emission_scale() { return NVB_EXP_SCALE; }
 
 // Doubles of global scratch the striped sweep needs for its hand-off rows (0 when they fit shared memory).
-int64_t nvbk_sweep2_global_handoff_doubles(int mode, int n_reads, int wave_maxw, int force_warps) {
-  const SweepPlan p = plan_sweep(mode, wave_maxw, force_warps);
+int64_t nvbk_sweep2_global_handoff_doubles(int mode, int n_reads, int wave_maxw) {
+  const SweepPlan p = plan_sweep(mode, wave_maxw);
   return p.global_handoff ? (int64_t)2 * n_reads * 2 * (p.NW + 1) * p.width : 0;
 }
 
 // wave_maxw: widest band row among the reads [b0, b1).  Returns -1 for an unsupported min_event_length, -2 when the
 // shared-memory reservation fails.
-int nvbk_sweep2(const ModelDev &M, const BatchDev &B, int mode, int b0, int b1, int wave_maxw, int force_warps,
+int nvbk_sweep2(const ModelDev &M, const BatchDev &B, int mode, int b0, int b1, int wave_maxw,
                 const int64_t *d_mat_base, double *pF, int32_t *pX, double *sF, int32_t *sX, double *g_handoff,
                 cudaStream_t st) {
   const int n_items = 2 * (b1 - b0);
   if (n_items <= 0) return 0;
-  const SweepPlan p = plan_sweep(mode, wave_maxw, force_warps);
+  const SweepPlan p = plan_sweep(mode, wave_maxw);
   if (p.global_handoff && g_handoff == nullptr) return -2;
   double *gh = p.global_handoff ? g_handoff : nullptr;
   const int NW = p.NW, width = p.width;

@@ -136,18 +136,6 @@ class Batch:
     def n_reads(self):
         return self.pack.n_reads
 
-    def set_signals(self, signals):
-        """Replace the signal values; `signals` is a list of per-read arrays or one flat float64 array."""
-        if isinstance(signals, np.ndarray) and signals.ndim == 1 and signals.dtype == np.float64:
-            flat = np.ascontiguousarray(signals)
-        else:
-            flat = np.ascontiguousarray(np.concatenate([np.asarray(s, dtype=np.float64) for s in signals])
-                                        if len(signals) else np.zeros(0), dtype=np.float64)
-        if flat.size != self.pack.total_signal:
-            raise ValueError('replacement signals must keep the batch layout')
-        _cabi.check(self.lib.nvb_batch_set_signal(self.handle, _cabi.ptr(flat, ctypes.c_double)),
-                    'nvb_batch_set_signal')
-
     def apply_splines(self, splines, stream=None):
         """Replace every read's resident signal x by spline(x); `splines` holds one FITPACK (t, c, k) tuple per read
         as returned by scipy.interpolate.splrep, or None to leave that read untouched."""
@@ -170,7 +158,7 @@ class Batch:
                                                      degree, _stream(stream)), 'nvb_batch_apply_splines')
 
     def signals(self):
-        """The resident signal values per read (after set_signals / apply_splines)."""
+        """The resident signal values per read (after apply_splines)."""
         out = np.zeros(self.pack.total_signal, dtype=np.float64)
         _cabi.check(self.lib.nvb_batch_get_signal(self.handle, _cabi.ptr(out, ctypes.c_double)), 'nvb_batch_get_signal')
         off = self.pack.signal_off
@@ -253,12 +241,6 @@ class Batch:
                                                     float(normalization_event_length), ctypes.c_void_p(d_chunks),
                                                     _stream(stream)), 'nvb_batch_chunk_values')
 
-    def scatter_add(self, d_chunks, dest, d_acc, d_cov, stream=None):
-        d = _cabi.as_array(dest, np.int64)
-        _cabi.check(self.lib.nvb_batch_scatter_add(self.handle, ctypes.c_void_p(d_chunks),
-                                                   _cabi.ptr(d, ctypes.c_int64), ctypes.c_void_p(d_acc),
-                                                   ctypes.c_void_p(d_cov), _stream(stream)), 'nvb_batch_scatter_add')
-
     def scatter_add_rows(self, d_chunks, dest, d_rows, stream=None):
         """Add the chunks into consensus rows of 5 doubles [A, C, G, T, coverage] (one buffer, one collective)."""
         d = _cabi.as_array(dest, np.int64)
@@ -324,23 +306,6 @@ def _stream(stream):
     if stream is None:
         return ctypes.c_void_p(0)
     return ctypes.c_void_p(int(getattr(stream, 'cuda_stream', stream)))
-
-
-def posterior(device, d_ll, d_ref, group_off, k, snp_prior, d_out, stream=None):
-    """_compute_posterior on the device over concatenated groups (pointers are device data pointers)."""
-    lib = _cabi.require_device()
-    g = _cabi.as_array(group_off, np.int64)
-    _cabi.check(lib.nvb_posterior(int(device), ctypes.c_void_p(d_ll), ctypes.c_void_p(d_ref),
-                                  _cabi.ptr(g, ctypes.c_int64), len(g) - 1, int(k), float(snp_prior),
-                                  ctypes.c_void_p(d_out), _stream(stream)), 'nvb_posterior')
-
-
-def posterior_resident(device, d_ll, d_ref, d_group_off, n_groups, total, k, snp_prior, d_out, stream=None):
-    """_compute_posterior with the group offsets already on the device: enqueues the kernel, no synchronisation."""
-    lib = _cabi.require_device()
-    _cabi.check(lib.nvb_posterior_d(int(device), ctypes.c_void_p(d_ll), ctypes.c_void_p(d_ref),
-                                    ctypes.c_void_p(d_group_off), int(n_groups), int(total), int(k), float(snp_prior),
-                                    ctypes.c_void_p(d_out), _stream(stream)), 'nvb_posterior_d')
 
 
 def posterior_rows(device, d_rows, base_row, row_lo, row_hi, d_ref, d_group_off, n_groups, k, snp_prior, d_out_rows,

@@ -296,15 +296,20 @@ class ProbabilityEstimator:
         return out
 
     def _compute_posterior(self, log_likelihoods, reference):
-        """estimator.py:131-156 for one group, on the device."""
+        """estimator.py:131-156 for one group, on the device: the log-likelihoods go through the consensus-row
+        posterior kernel as a group of rows of 5 doubles (coverage column 0)."""
         import torch
         dev = _device(self.kmer_model)
-        ll = torch.as_tensor(numpy.ascontiguousarray(log_likelihoods, dtype=numpy.float64), device=dev)
+        ll = torch.as_tensor(numpy.asarray(log_likelihoods, dtype=numpy.float64), device=dev)
+        L = ll.shape[0]
+        rows = torch.zeros((L, 5), dtype=torch.float64, device=dev)
+        rows[:, :4] = ll
         ref = torch.as_tensor(_ref_codes(reference), device=dev)
-        out = torch.empty_like(ll)
-        dtw.posterior(dev.index, ll.data_ptr(), ref.data_ptr(), [0, ll.shape[0]], self.kmer_model.get_k(),
-                      self.snp_prior, out.data_ptr(), torch.cuda.current_stream())
-        return out.cpu().numpy()
+        group_off = torch.tensor([0, L], dtype=torch.int64, device=dev)
+        out = torch.empty_like(rows)
+        dtw.posterior_rows(dev.index, rows.data_ptr(), 0, 0, L, ref.data_ptr(), group_off.data_ptr(), 1,
+                           self.kmer_model.get_k(), self.snp_prior, out.data_ptr(), torch.cuda.current_stream())
+        return out[:, :4].cpu().numpy()
 
     def estimate_probabilities(self, reference, reads, independent=False, process_group=None):
         """estimator.py:199-236.  `independent=True` treats every read as its own group (what estimate_snps does

@@ -26,7 +26,7 @@ def test_header_declares_the_boundary():
     names = declared_functions()
     for must in ('nvb_model_create', 'nvb_model_expected_signal', 'nvb_refine_alignment_batch',
                  'nvb_estimate_log_likelihoods_batch', 'nvb_batch_create', 'nvb_batch_refine', 'nvb_batch_estimate',
-                 'nvb_posterior', 'nvb_batch_scatter_add', 'nvb_last_error'):
+                 'nvb_posterior_rows_d', 'nvb_batch_scatter_add_rows', 'nvb_last_error'):
         assert must in names
     # every entry point cites the reference interface it replaces
     text = open(HEADER).read()

@@ -14,8 +14,9 @@ int64 exponent, about 2^-64 per operation whatever the magnitude), and the bars 
      within 64 eps (row + column depth) in log;
   c. chunk_values_kernel: bit-exact against numpy on the GPU's own raw LLs;
   d. scatter_add_rows_kernel: |GPU - fsum| <= (m - 1) eps sum|x| for m summands (any summation order), coverage exact;
-  e. posterior_kernel / posterior_rows_kernel: rtol 1e-13 against 50-digit mpmath on the GPU's own input rows; 0/0
-     rows of the reference's double arithmetic are NaN; a halo slice is bit-identical to the unsliced call;
+  e. posterior_rows_kernel, directly and through ProbabilityEstimator._compute_posterior: rtol 1e-13 against 50-digit
+     mpmath on the GPU's own input rows; 0/0 rows of the reference's double arithmetic are NaN; a halo slice is
+     bit-identical to the unsliced call;
   f. ProbabilityEstimator.estimate_probabilities, consensus and independent, against extended ratios -> long double
      chunks -> fsum -> 50-digit posterior: rtol 1e-8 on probabilities >= 1e-12, 1e-15 below; coverage exact.
 
@@ -431,14 +432,16 @@ def _nan_rows(ll, ref, group_off, k, prior):
 
 
 @pytest.mark.gpu
-def test_posterior_kernels_match_mpmath(lib_built):
-    """Part e: posterior_kernel and posterior_rows_kernel at k 1, 2, 6, 11 and snp_prior 0.001, 0.3 against 50-digit
-    mpmath, rtol 1e-13 (atol 1e-290 for probabilities the double exp leaves subnormal); the 0/0 rows NaN.  Halo slices
-    [row_lo, row_hi) -- every group boundary and seeded random ones -- from a buffer that starts at row_lo - (k-1) (the
-    group start when row_lo opens one) and is NaN outside the rows the window can reach: bit-identical to the unsliced
-    call, coverage column included."""
+def test_posterior_rows_match_mpmath(lib_built):
+    """Part e: posterior_rows_kernel, called directly and through ProbabilityEstimator._compute_posterior once per
+    group, at k 1, 2, 6, 11 and snp_prior 0.001, 0.3 against 50-digit mpmath, rtol 1e-13 (atol 1e-290 for
+    probabilities the double exp leaves subnormal); the 0/0 rows NaN.  Halo slices [row_lo, row_hi) -- every group
+    boundary and seeded random ones -- from a buffer that starts at row_lo - (k-1) (the group start when row_lo opens
+    one) and is NaN outside the rows the window can reach: bit-identical to the unsliced call, coverage column
+    included."""
     import torch
     from nadavca_b200 import dtw
+    from nadavca_b200.estimator import ProbabilityEstimator
     dev = torch.cuda.current_device()
     worst = 0.0
     nan_rows_seen = 0
@@ -449,19 +452,20 @@ def test_posterior_kernels_match_mpmath(lib_built):
             truth = _mp_posterior(ll, ref, goff, k, prior)
             nan_rows = _nan_rows(ll, ref, goff, k, prior)
             nan_rows_seen += int(nan_rows.sum())
-            d_ll = torch.as_tensor(ll, device='cuda')
+            # _compute_posterior reads only k and the device of its model: constant tables, no model on the device
+            km = dtw.KmerModel(k, 0, 4, np.zeros(4 ** k), np.ones(4 ** k), device=dev)
+            est = ProbabilityEstimator(km, None, dict(E2E_CONFIG, snp_prior_probability=prior))
+            p4 = np.concatenate([est._compute_posterior(ll[gs:ge], ref[gs:ge]) for gs, ge in zip(goff[:-1], goff[1:])])
             d_ref = torch.as_tensor(ref, device='cuda')
             d_goff = torch.as_tensor(goff, device='cuda')
-            out4 = torch.empty((total, 4), dtype=torch.float64, device='cuda')
-            dtw.posterior(dev, d_ll.data_ptr(), d_ref.data_ptr(), goff, k, prior, out4.data_ptr())
             rows = torch.as_tensor(np.concatenate([ll, cov[:, None]], axis=1), device='cuda')
             full = torch.empty((total, 5), dtype=torch.float64, device='cuda')
             dtw.posterior_rows(dev, rows.data_ptr(), 0, 0, total, d_ref.data_ptr(), d_goff.data_ptr(), len(goff) - 1,
                                k, prior, full.data_ptr())
             torch.cuda.synchronize()
-            p4, p5 = out4.cpu().numpy(), full.cpu().numpy()
+            p5 = full.cpu().numpy()
             assert np.array_equal(p5[:, 4], cov)
-            for got, name in ((p4, 'posterior'), (p5[:, :4], 'posterior_rows')):
+            for got, name in ((p4, '_compute_posterior'), (p5[:, :4], 'posterior_rows')):
                 assert np.array_equal(np.isnan(got).any(axis=1), nan_rows), '%s k %d prior %g: NaN rows' % (name, k,
                                                                                                              prior)
                 ok = ~nan_rows

@@ -554,7 +554,7 @@ def test_thresholds_pinned_to_sources():
     m = re.search(r'bool rotate = w\.maxw <= (\d+) && \(w\.maxw <= (\d+) \|\| mode == NVB_MODE_PLAIN \|\| '
                   r'4 \* items >= resident\);', api)
     assert m and (int(m.group(1)), int(m.group(2))) == (ROT_MAX, ROT_ONE_SLOT)
-    assert re.search(r'rotate = w\.maxw <= %d && g_opt\.sweep == NVB_SWEEP_ROTATE;' % ROT_MAX, api)
+    assert re.search(r'rotate = w\.maxw <= %d && g_sweep == NVB_SWEEP_ROTATE;' % ROT_MAX, api)
     assert re.search(r'const int items = 2 \* \(w\.b1 - w\.b0\);', api)
     assert int(re.search(r'const int resident = b->model->sm_count \* (\d+);', api).group(1)) == ROT_WARPS_PER_SM
     assert re.search(r'rotate = !b->no_rotation\[i\];', api)
